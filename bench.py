@@ -14,6 +14,10 @@ Prints ONE JSON line (rank 0).  `value` = images/s with the batch already reside
 `e2e` = the same step fed from pinned HOST buffers (H2D of images+labels and D2H of the loss inside
 the timed region).  `--impl reference` times the reference's own CPU implementation of the same
 step on the host cores (tools/cpu_reference.py) and prints the same line with "impl": "reference".
+
+`--dump-outputs DIR` writes what the last resident timed step computed (rank 0) as DIR/<name>.npy, so that two
+builds run with the same arguments, hence the same inputs, can be compared output for output (dump_outputs below).
+The bench writes nothing into the source tree.
 """
 import argparse
 import json
@@ -24,6 +28,8 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True                 # the tree may be read-only; keep it untouched either way
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"    # the CPU baseline's worker processes
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
@@ -183,6 +189,31 @@ def conv_roofline(torch, lib, peaks, peak_kind, iters=10):
                 "tcgen05-tf32": "the kernel multiplies in tf32, whose tensor peak is half of bf16"}.get(path, path))}
 
 
+DUMP_SAMPLE = 1 << 22       # elements kept of a larger output: parameters and gradients are sampled (16 MB each)
+
+
+def dump_outputs(torch, net, out_dir):
+    """What the training step hands back, after the last timed step: the output layer's softmax probabilities, the summed
+    cross-entropy of the batch, the updated parameters and their gradients.  Parameters and gradients are the same fixed,
+    seeded sample of DUMP_SAMPLE positions inside the edges (never the padding between them); float32 .npy files."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    edges = [(off, size) for _, _, off, size in net.edges() if size > 0]
+    offs, sizes = np.array([o for o, _ in edges], np.int64), np.array([s for _, s in edges], np.int64)
+    starts = np.cumsum(sizes) - sizes
+    total = int(sizes.sum())
+    pick = np.unique(np.random.RandomState(0).randint(0, total, DUMP_SAMPLE)) if total > DUMP_SAMPLE else np.arange(total)
+    e = np.searchsorted(starts, pick, side="right") - 1
+    params = net.params_tensor()
+    idx = torch.from_numpy(offs[e] + (pick - starts[e])).to(params.device)
+    out = {"output": net.output_tensor().cpu().numpy(),
+           "loss": np.array([net.loss()], np.float32),
+           "params_sample": params[idx].cpu().numpy(),
+           "grads_sample": net.grads_tensor()[idx].cpu().numpy()}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -196,7 +227,10 @@ def main():
     ap.add_argument("--no-prefetch", action="store_true", help="e2e: copy each batch synchronously instead of one step ahead")
     ap.add_argument("--bucket-mb", type=float, default=128.0, help="gradient all-reduce bucket size")
     ap.add_argument("--no-cfg3", action="store_true", help="N > 1: skip the extra 256-images-per-GPU measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -293,6 +327,8 @@ def main():
     ms_total = timed(step_resident, args.steps)
     sampler.window(t0, time.time())
     launches = int(L.convnet_b200_launch_count())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, net, args.dump_outputs)
     ev_consumed.record()
     prefetch()                                               # the first timed step's batch
     for _ in range(2):

@@ -90,6 +90,36 @@ def build_host(force=False):
     return HOST_LIB
 
 
+ROOT = os.path.dirname(HERE)
+DROP_IN_SRC = os.path.join(ROOT, "tests", "drop_in", "link_drop_in.cc")
+DROP_IN_BIN = os.path.join(ROOT, "tests", "drop_in", "_build", "link_drop_in")
+
+
+def reference_headers():
+    """the reference's cudamat/ header directory, when CONVNET_REFERENCE names the reference's source tree"""
+    ref = os.environ.get("CONVNET_REFERENCE")
+    return os.path.join(ref, "cudamat") if ref and os.path.isdir(os.path.join(ref, "cudamat")) else None
+
+
+def build_drop_in(ref_headers=None):
+    """the link-level drop-in program (tests/drop_in), twice: linked with -lcudamat_conv_gemm only and with
+    -lcudamat_conv only (both names are aliases of the one product library, so either must resolve BOTH symbol sets the
+    program calls); rpath points at convnet_b200/lib relative to the binary.  It is compiled against the reference's own
+    headers from `ref_headers` when given, else against the project's declarations of the same two ABIs (include/)."""
+    libdir = os.path.dirname(build())
+    os.makedirs(os.path.dirname(DROP_IN_BIN), exist_ok=True)
+    headers = ["-I" + ref_headers] if ref_headers else ["-DDROP_IN_OWN_HEADERS", "-I" + os.path.join(ROOT, "include")]
+    outs = []
+    for alias in ("cudamat_conv_gemm", "cudamat_conv"):
+        out = DROP_IN_BIN + "_" + alias
+        cmd = ["g++", "-O1", "-std=c++14"] + headers + ["-I/usr/local/cuda/include", DROP_IN_SRC, "-o", out,
+               "-L" + libdir, "-l" + alias, "-L/usr/local/cuda/lib64", "-lcudart",
+               "-Wl,--no-undefined", "-Wl,-rpath,$ORIGIN/../../../convnet_b200/lib", "-Wl,-rpath,/usr/local/cuda/lib64"]
+        subprocess.run(cmd, check=True)
+        outs.append(out)
+    return outs
+
+
 if __name__ == "__main__":
     build_host(force="--force" in sys.argv)
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

@@ -17,11 +17,3 @@ def oracle():
     from oracle_lib import Oracle, build_oracle
     build_oracle()
     return Oracle()
-
-
-@pytest.fixture(scope="session")
-def reflib():
-    from oracle_lib import RefLib
-    if not RefLib.available():
-        pytest.skip("oracle/_ref/libeigenmat_ref.so not built (needs /root/reference)")
-    return RefLib()

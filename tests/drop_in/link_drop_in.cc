@@ -5,7 +5,8 @@
 // itself, and is linked with `-lcudamat_conv_gemm -lcudamat_conv` resolved from convnet_b200/lib — the two library
 // names the reference's Makefile:72-77 links.  If a prototype, a struct layout or a symbol name of the product
 // differed from the reference's, this file would fail to compile, to link, or to compute the right numbers.
-// Built by tests/test_link_drop_in.py / __graft_entry__.build() where /root/reference exists; run on the GPU box.
+// Without the reference's headers (DROP_IN_OWN_HEADERS) it includes the project's declarations of the same two ABIs,
+// and still proves the library names, both symbol sets and the numbers.  Built by convnet_b200/build.py build_drop_in.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -13,8 +14,13 @@
 #include <cstdlib>
 #include <vector>
 
+#ifdef DROP_IN_OWN_HEADERS
+#include "convnet_b200_conv_gemm.h"
+#include "convnet_b200_conv.h"
+#else
 #include "cudamat_conv_gemm.cuh"   // the reference's ABI-1 header (pulls in cudamat.cuh: cudamat, Shape4D, ConvDesc)
 #include "cudamat_conv.cuh"        // the reference's ABI-2 header
+#endif
 
 static void ck(cudaError_t e, const char* what) {
   if (e != cudaSuccess) { fprintf(stderr, "%s: %s\n", what, cudaGetErrorString(e)); exit(2); }

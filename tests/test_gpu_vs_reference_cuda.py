@@ -1,9 +1,12 @@
 """BASELINE-size parity on the GPU against the REFERENCE'S OWN CUDA KERNELS.
 
-oracle/_ref/libcudamat_conv_gemm_ref.so is cudamat/cudamat_conv_gemm.cu + cudamat_conv3d_gemm.cu compiled unmodified
-for sm_100 (oracle/Makefile).  Every layer of net A (examples/imagenet/CLS_net_20140801232522.pbtxt, SURVEY.md
-Appendix B) at batch 128 (BASELINE config 2) and 256 (config 3), and the cfg4 C3D conv1a / conv2a shapes at batch 32,
-runs through BOTH libraries on identical seeded inputs: fprop / dgrad / wgrad, pool1/2/5 (+undo), rnorm1/2 (+undo).
+The reference side is cudamat/cudamat_conv_gemm.cu + cudamat_conv3d_gemm.cu compiled unmodified for sm_100
+(oracle/Makefile -> oracle/_ref/libcudamat_conv_gemm_ref.so); what it computed is stored in tests/golden/ref_cuda.npz
+(tests/golden_ref.py: seeded samples, and a digest of every output that must match bit for bit), recorded on a B200 with
+CONVNET_B200_RECORD_GOLDEN=1, which runs the reference live.  Every layer of net A
+(examples/imagenet/CLS_net_20140801232522.pbtxt, SURVEY.md Appendix B) at batch 128 (BASELINE config 2) and 256
+(config 3), and the cfg4 C3D conv1a / conv2a shapes at batch 32, runs on identical seeded inputs (the CUDA generator):
+fprop / dgrad / wgrad, pool1/2/5 (+undo), rnorm1/2 (+undo).
 
 Metric and tolerances are the ones of tests/test_gpu_parity.py: Diff = max|a-b| / mean|a+b| (py/test_conv.py:382-385);
 fp32 mode 1e-4 (the reference's own bar), tf32 5e-3, bf16 2.5e-2; max-pool values bit-exact; pool-undo / rnorm 1e-4, rnorm
@@ -16,6 +19,7 @@ import zlib
 import numpy as np
 import pytest
 
+import golden_ref
 import ref_cuda_lib
 from convnet_b200.abi import GetConvDesc, num_modules
 
@@ -31,8 +35,8 @@ _RESULTS = {}
 def env():
     import torch
     assert torch.cuda.is_available(), "these tests need a CUDA device"
-    if not ref_cuda_lib.available():
-        pytest.fail("oracle/_ref/libcudamat_conv_gemm_ref.so is missing: run `make -C oracle` where /root/reference exists")
+    if golden_ref.RECORD and not ref_cuda_lib.available():
+        pytest.fail("recording needs oracle/_ref/libcudamat_conv_gemm_ref.so: run `make -C oracle` where the reference exists")
     from convnet_b200 import conv_gemm as cg
     from convnet_b200 import lib
     from convnet_b200.matrix import CUDAMatrix
@@ -41,7 +45,9 @@ def env():
     class E:
         pass
     e = E()
-    e.torch, e.lib, e.ours, e.ref, e.M = torch, lib, cg.gemm, ref_cuda_lib.binding(), CUDAMatrix
+    e.torch, e.lib, e.ours, e.M = torch, lib, cg.gemm, CUDAMatrix
+    store = golden_ref.RefStore("ref_cuda")
+    ref_api = ref_cuda_lib.binding() if golden_ref.RECORD else None
 
     def rand(rows, cols, s4, gen, scale=1.0, uniform=False):
         m = CUDAMatrix(rows, cols, s4)
@@ -58,16 +64,29 @@ def env():
         m.fill_(float("nan"))
         return m
     e.rand, e.nan = rand, nan
-    e.zeros = lambda rows, cols, s4: CUDAMatrix(rows, cols, s4)      # reference targets (not the object under test)
+
+    def ref(key, rows, cols, s4, call, init=None, exact=False):
+        """the reference's result of call(api, target) on a zero (or `init`) target: live when recording, else stored"""
+        def compute():
+            m = CUDAMatrix(rows, cols, s4)
+            if init is not None:
+                m.storage.copy_(init.storage)
+            call(ref_api, m)
+            torch.cuda.synchronize()
+            return m.storage
+        return store.reference(key, compute, exact)
+    e.ref = ref
 
     def diff(a, b):
-        a, b = a.storage, b.storage
-        assert torch.isfinite(a).all() and torch.isfinite(b).all()
-        num = (a - b).abs().max().item()
-        den = (a + b).abs().mean(dtype=torch.float64).item()
-        return num / den if den > 0 else num
+        a = a.storage
+        assert torch.isfinite(a).all()
+        if not isinstance(b, golden_ref.Stored):
+            assert torch.isfinite(b).all()
+        return golden_ref.diff(a, b)
     e.diff = diff
+    e.equal = lambda a, b: golden_ref.equal(a.storage, b)
     yield e
+    store.save()
     lib.set_precision("tf32")
     out = os.path.join(ROOT, "gpurun_out")
     os.makedirs(out, exist_ok=True)
@@ -108,10 +127,10 @@ def test_alexnet_conv_layers(env, layer, N):
     w = env.rand(Cout, K, fsh, g, scale=1.0 / np.sqrt(K))
     dv = env.rand(N, modX * modY * Cout, tsh, g)
     # the reference, once
-    r_up = env.zeros(N, modX * modY * Cout, tsh); env.ref.convUp(x, w, r_up, d, 0)
-    r_dn = env.zeros(N, W * H * Cin, ish); env.ref.convDown(dv, w, r_dn, d, 0)
-    r_dw = env.zeros(Cout, K, fsh); env.ref.convOutp(x, dv, r_dw, d, 0, 1.0 / N)
-    torch.cuda.synchronize()
+    key = "%s_b%d/" % (layer, N)
+    r_up = env.ref(key + "fprop", N, modX * modY * Cout, tsh, lambda api, t: api.convUp(x, w, t, d, 0))
+    r_dn = env.ref(key + "dgrad", N, W * H * Cin, ish, lambda api, t: api.convDown(dv, w, t, d, 0))
+    r_dw = env.ref(key + "wgrad", Cout, K, fsh, lambda api, t: api.convOutp(x, dv, t, d, 0, 1.0 / N))
     for mode in ("fp32", "tf32", "bf16"):
         env.lib.set_precision(mode)
         out = env.nan(N, modX * modY * Cout, tsh); env.ours.convUp(x, w, out, d, 0); p_up = env.lib.last_conv_path()
@@ -145,7 +164,10 @@ def test_alexnet_conv_accumulate(env, N):
         b = env.M(N, W * H * Cin, ish); b.storage.copy_(i_dn.storage); api.convDown(dv, w, b, d, 1)
         c = env.M(Cout, K, fsh); c.storage.copy_(i_dw.storage); api.convOutp(x, dv, c, d, 1, 0.5)
         return a, b, c
-    ref = run(env.ref)
+    key = "conv3_accum_b%d/" % N
+    ref = (env.ref(key + "fprop", N, 196 * Cout, tsh, lambda api, t: api.convUp(x, w, t, d, 1), init=i_up),
+           env.ref(key + "dgrad", N, W * H * Cin, ish, lambda api, t: api.convDown(dv, w, t, d, 1), init=i_dn),
+           env.ref(key + "wgrad", Cout, K, fsh, lambda api, t: api.convOutp(x, dv, t, d, 1, 0.5), init=i_dw))
     for mode in ("fp32", "tf32", "bf16"):
         env.lib.set_precision(mode)
         for name, a, b in zip(("fprop", "dgrad", "wgrad"), run(env.ours), ref):
@@ -169,19 +191,21 @@ def test_alexnet_pool_layers(env, layer, N):
     x = env.rand(N, W * W * C, ish, g)
     gr = env.rand(N, mod * mod * C, psh, g)
     res = {}
-    r_mx = env.zeros(N, mod * mod * C, psh); env.ref.MaxPool(x, r_mx, d)
+    key = "%s_b%d/" % (layer, N)
+    r_mx = env.ref(key + "max", N, mod * mod * C, psh, lambda api, t: api.MaxPool(x, t, d), exact=True)
     o_mx = env.nan(N, mod * mod * C, psh); env.ours.MaxPool(x, o_mx, d)
-    assert torch.equal(r_mx.storage, o_mx.storage), "max-pool values must be bit-exact"
-    r_av = env.zeros(N, mod * mod * C, psh); env.ref.AvgPool(x, r_av, d)
+    assert env.equal(o_mx, r_mx), "max-pool values must be bit-exact"
+    r_av = env.ref(key + "avg", N, mod * mod * C, psh, lambda api, t: api.AvgPool(x, t, d))
     o_av = env.nan(N, mod * mod * C, psh); env.ours.AvgPool(x, o_av, d)
     res["avg"] = env.diff(o_av, r_av)
     for st in (0, 1):
         init = env.rand(N, W * W * C, ish, g)
-        r = env.M(N, W * W * C, ish); r.storage.copy_(init.storage); env.ref.MaxPoolUndo(x, gr, r_mx, r, d, st)
+        r = env.ref(key + "max_undo_st%d" % st, N, W * W * C, ish,
+                    lambda api, t: api.MaxPoolUndo(x, gr, env.M(N, mod * mod * C, psh, storage=r_mx), t, d, st), init=init)
         o = env.M(N, W * W * C, ish); o.storage.copy_(init.storage if st else torch.full_like(init.storage, float("nan")))
         env.ours.MaxPoolUndo(x, gr, o_mx, o, d, st)
         res["max_undo_st%d" % st] = env.diff(o, r)
-        r = env.M(N, W * W * C, ish); r.storage.copy_(init.storage); env.ref.AvgPoolUndo(gr, r, d, st)
+        r = env.ref(key + "avg_undo_st%d" % st, N, W * W * C, ish, lambda api, t: api.AvgPoolUndo(gr, t, d, st), init=init)
         o = env.M(N, W * W * C, ish); o.storage.copy_(init.storage if st else torch.full_like(init.storage, float("nan")))
         env.ours.AvgPoolUndo(gr, o, d, st)
         res["avg_undo_st%d" % st] = env.diff(o, r)
@@ -203,10 +227,12 @@ def test_alexnet_rnorm_layers(env, layer, N):
     x, dy = env.rand(N, W * W * C, ish, g), env.rand(N, W * W * C, ish, g)
     res = {}
     for blocked in (False, True):
-        r = env.zeros(N, W * W * C, ish); env.ref.ResponseNormCrossMap(x, r, k, 5e-4, 0.75, blocked)
+        key = "%s_b%d/blocked%d_" % (layer, N, blocked)
+        r = env.ref(key + "fwd", N, W * W * C, ish, lambda api, t: api.ResponseNormCrossMap(x, t, k, 5e-4, 0.75, blocked))
         o = env.nan(N, W * W * C, ish); env.ours.ResponseNormCrossMap(x, o, k, 5e-4, 0.75, blocked)
         res["fwd_blocked%d" % blocked] = env.diff(o, r)
-        r = env.zeros(N, W * W * C, ish); env.ref.ResponseNormCrossMapUndo(dy, x, r, k, 5e-4, 0.75, blocked)
+        r = env.ref(key + "undo", N, W * W * C, ish,
+                    lambda api, t: api.ResponseNormCrossMapUndo(dy, x, t, k, 5e-4, 0.75, blocked))
         o = env.nan(N, W * W * C, ish); env.ours.ResponseNormCrossMapUndo(dy, x, o, k, 5e-4, 0.75, blocked)
         res["undo_blocked%d" % blocked] = env.diff(o, r)
     _RESULTS["%s_b%d" % (layer, N)] = res
@@ -235,10 +261,10 @@ def test_c3d_conv_layers(env, layer):
     x = env.rand(N, W * W * Cin * T, ish, g)
     w = env.rand(Cout, K, fsh, g, scale=1.0 / np.sqrt(K))
     dv = env.rand(N, W * W * Cout * To, tsh, g)
-    r_up = env.zeros(N, W * W * Cout * To, tsh); env.ref.convUp3D(x, w, r_up, d, 0)
-    r_dn = env.zeros(N, W * W * Cin * T, ish); env.ref.convDown3D(dv, w, r_dn, d, 0)
-    r_dw = env.zeros(Cout, K, fsh); env.ref.convOutp3D(x, dv, r_dw, d, 0, 1.0 / N)
-    torch.cuda.synchronize()
+    key = "c3d_%s_b%d/" % (layer, N)
+    r_up = env.ref(key + "fprop", N, W * W * Cout * To, tsh, lambda api, t: api.convUp3D(x, w, t, d, 0))
+    r_dn = env.ref(key + "dgrad", N, W * W * Cin * T, ish, lambda api, t: api.convDown3D(dv, w, t, d, 0))
+    r_dw = env.ref(key + "wgrad", Cout, K, fsh, lambda api, t: api.convOutp3D(x, dv, t, d, 0, 1.0 / N))
     for mode in ("fp32", "tf32", "bf16"):
         env.lib.set_precision(mode)
         out = env.nan(N, W * W * Cout * To, tsh); env.ours.convUp3D(x, w, out, d, 0); p_up = env.lib.last_conv_path()
@@ -263,10 +289,11 @@ def test_c3d_pool_layer(env):
     g = torch.Generator(device="cuda").manual_seed(3)
     x = env.rand(N, W * W * C * T, ish, g)
     gr = env.rand(N, (W // 2) ** 2 * C * (T // 2), psh, g)
-    r_mx = env.zeros(gr.rows, gr.cols, psh); env.ref.MaxPool(x, r_mx, d)
+    r_mx = env.ref("c3d_pool2_b32/max", gr.rows, gr.cols, psh, lambda api, t: api.MaxPool(x, t, d), exact=True)
     o_mx = env.nan(gr.rows, gr.cols, psh); env.ours.MaxPool(x, o_mx, d)
-    assert torch.equal(r_mx.storage, o_mx.storage)
-    r = env.zeros(x.rows, x.cols, ish); env.ref.MaxPoolUndo(x, gr, r_mx, r, d, 0)
+    assert env.equal(o_mx, r_mx)
+    r = env.ref("c3d_pool2_b32/max_undo", x.rows, x.cols, ish,
+                lambda api, t: api.MaxPoolUndo(x, gr, env.M(gr.rows, gr.cols, psh, storage=r_mx), t, d, 0))
     o = env.nan(x.rows, x.cols, ish); env.ours.MaxPoolUndo(x, gr, o_mx, o, d, 0)
     dd = env.diff(o, r)
     _RESULTS["c3d_pool2_b32"] = {"max_undo": dd}

@@ -1,11 +1,13 @@
 """SURVEY.md §8 f4, device side: the minibatch crop / mirror / transpose (convnet_b200_extract_patches) — the oracle pinned
-to the reference's own CPU implementation (eigenmat/eigenmat.cc:2046-2090), the C-ABI's argument checks, and (GPU) the
-kernel against the oracle, bit for bit."""
+to the reference's own CPU implementation (eigenmat/eigenmat.cc:2046-2090; its results stored in
+tests/golden/ref_eigenmat_patches.npz, see tests/golden_ref.py), the C-ABI's argument checks, and (GPU) the kernel against
+the oracle, bit for bit."""
 import ctypes as ct
 
 import numpy as np
 import pytest
 
+import golden_ref
 from oracle_lib import Oracle, RefLib
 
 CASES = [  # N, C, W, H, pw, ph
@@ -36,18 +38,29 @@ def _numpy_reference(images, wo, ho, flip, N, C, W, H, pw, ph):
     return out.reshape(-1)
 
 
+@pytest.fixture(scope="module")
+def ref_patches():
+    """stored results of the reference's CPU code; recording runs it live (oracle/_ref/libeigenmat_ref.so)"""
+    store = golden_ref.RefStore("ref_eigenmat_patches")
+    if golden_ref.RECORD and not (RefLib.available() and hasattr(RefLib().lib, "ref_extract_patches")):
+        pytest.fail("recording needs oracle/_ref/libeigenmat_ref.so with the extract_patches door: run `make -C oracle`")
+    yield store
+    store.save()
+
+
 @pytest.mark.parametrize("case", CASES)
-def test_oracle_equals_the_formula_and_the_reference_cpu_code(case):
+def test_oracle_equals_the_formula_and_the_reference_cpu_code(case, ref_patches):
     N, C, W, H, pw, ph = case
     images, wo, ho, flip = _inputs(*case, seed=3)
     got = np.asfortranarray(np.full(N * C * pw * ph, np.nan, np.float32))
     assert Oracle().extract_patches(images, got, wo, ho, flip, N, C, W, H, pw, ph) == 0
     assert np.array_equal(got, _numpy_reference(images, wo, ho, flip, N, C, W, H, pw, ph))
-    if not RefLib.available() or not hasattr(RefLib().lib, "ref_extract_patches"):
-        pytest.skip("oracle/_ref/libeigenmat_ref.so (with the extract_patches door) not built")
-    ref = np.asfortranarray(np.full(N * C * pw * ph, np.nan, np.float32))
-    assert RefLib().extract_patches(images, ref, wo, ho, flip, N, C, W, H, pw, ph) == 0
-    assert np.array_equal(got, ref)
+
+    def live():
+        ref = np.asfortranarray(np.full(N * C * pw * ph, np.nan, np.float32))
+        assert RefLib().extract_patches(images, ref, wo, ho, flip, N, C, W, H, pw, ph) == 0
+        return ref
+    assert golden_ref.equal(got, ref_patches.reference("x".join(map(str, case)), live, exact=True))
 
 
 def test_argument_checks_return_the_reference_error_code():

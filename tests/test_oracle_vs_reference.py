@@ -1,12 +1,14 @@
 """Pin oracle/conv_oracle.c (CPU, no GPU) against
   (a) the golden vectors produced by the reference's py/conv_cpu.py (tools/gen_golden.py), and
-  (b) the reference's compiled CPU library oracle/_ref/libeigenmat_ref.so (eigenmat/cpumat_conv.cc).
+  (b) the reference's compiled CPU library (eigenmat/cpumat_conv.cc built into oracle/_ref/libeigenmat_ref.so), whose
+      results are stored in tests/golden/ref_eigenmat.npz (tests/golden_ref.py).
 Metric and tolerance are the reference's own: Diff < 1e-4 (py/test_conv.py:382-392)."""
 import numpy as np
 import pytest
 
+import golden_ref
 from cases import F, GOLDEN_2D, GOLDEN_3D, Z, geo2d, geo3d, load_golden
-from oracle_lib import Diff
+from oracle_lib import Diff, RefLib
 
 TOL = 1e-4
 
@@ -83,6 +85,27 @@ def test_oracle_3d_vs_python_reference(oracle, name):
 
 
 # ---- (b) the reference's compiled CPU library ------------------------------------------------
+@pytest.fixture(scope="module")
+def reflib():
+    """(stored results, live library): the library only while recording (tests/golden_ref.py)"""
+    store = golden_ref.RefStore("ref_eigenmat")
+    if golden_ref.RECORD and not RefLib.available():
+        pytest.fail("recording needs oracle/_ref/libeigenmat_ref.so: run `make -C oracle` where the reference exists")
+    yield store, RefLib() if golden_ref.RECORD else None
+    store.save()
+
+
+def _reference(reflib, key, init, run, exact=True):
+    """what run(library, target) leaves in a copy of `init` (live when recording, else stored)"""
+    store, lib = reflib
+
+    def live():
+        b = init.copy(order="F")
+        run(lib, b)
+        return b
+    return store.reference(key, live, exact)
+
+
 CONV_SHAPES = [
     # N, W, H, Cin, Cout, ky, kx, sy, sx, py, px
     (16, 12, 12, 32, 64, 3, 3, 2, 2, 1, 1),      # py/test_conv.py 2-D geometry
@@ -109,10 +132,11 @@ def test_oracle_conv_bit_exact_vs_compiled_reference(oracle, reflib, shape, scal
             ("convDown", (derivs, filters, tsh, fsh, ish), (N, W * H * Cin)),
             ("convOutp", (images, derivs, ish, tsh, fsh), (Cout, kx * ky * Cin))):
         init = F(r.randn(*oshape))
-        a, b = init.copy(order="F"), init.copy(order="F")
+        a = init.copy(order="F")
         getattr(oracle, op)(args[0], args[1], a, *args[2:], d, scaleTargets, 0.5)
-        getattr(reflib, op)(args[0], args[1], b, *args[2:], d, scaleTargets, 0.5)
-        assert np.array_equal(a, b), (op, Diff(a, b))
+        key = "conv_%s_st%g/%s" % ("x".join(map(str, shape)), scaleTargets, op)
+        b = _reference(reflib, key, init, lambda lib, b: getattr(lib, op)(args[0], args[1], b, *args[2:], d, scaleTargets, 0.5))
+        assert golden_ref.equal(a, b), (op, golden_ref.diff(a, b))
 
 
 def test_oracle_channel_subrange_vs_compiled_reference(oracle, reflib):
@@ -127,10 +151,11 @@ def test_oracle_channel_subrange_vs_compiled_reference(oracle, reflib):
                              ("convDown", (derivs, filters, tsh, fsh, ish), (N, 64 * Cin)),
                              ("convOutp", (images, derivs, ish, tsh, fsh), (8, 54))):
         init = F(r.randn(*oshape))
-        a, b = init.copy(order="F"), init.copy(order="F")
+        a = init.copy(order="F")
         getattr(oracle, op)(args[0], args[1], a, *args[2:], d, 1.0, 1.0)
-        getattr(reflib, op)(args[0], args[1], b, *args[2:], d, 1.0, 1.0)
-        assert np.array_equal(a, b), op
+        b = _reference(reflib, "channel_subrange/" + op, init,
+                       lambda lib, b: getattr(lib, op)(args[0], args[1], b, *args[2:], d, 1.0, 1.0))
+        assert golden_ref.equal(a, b), op
 
 
 @pytest.mark.parametrize("F_sizeF", [(32, 8), (96, 24), (7, 3), (16, 16)])
@@ -139,9 +164,13 @@ def test_oracle_rnorm_bit_exact_vs_compiled_reference(oracle, reflib, F_sizeF, b
     nf, sizeF = F_sizeF
     r = np.random.RandomState(11)
     x, dy = F(r.randn(6, 5 * 5 * nf)), F(r.randn(6, 5 * 5 * nf))
-    a, b = Z(*x.shape), Z(*x.shape)
-    oracle.rnorm(x, a, nf, sizeF, 0.005, 0.75, blocked); reflib.rnorm(x, b, nf, sizeF, 0.005, 0.75, blocked)
-    assert Diff(a, b) < 1e-6
+    key = "rnorm_%d_%d_blocked%d/" % (nf, sizeF, blocked)
+    a = Z(*x.shape)
+    oracle.rnorm(x, a, nf, sizeF, 0.005, 0.75, blocked)
+    b = _reference(reflib, key + "fwd", Z(*x.shape), lambda lib, b: lib.rnorm(x, b, nf, sizeF, 0.005, 0.75, blocked),
+                   exact=False)
+    assert golden_ref.diff(a, b) < 1e-6
     oracle.rnormUndo(dy, x, a, nf, sizeF, 0.005, 0.75, blocked)
-    reflib.rnormUndo(dy, x, b, nf, sizeF, 0.005, 0.75, blocked)
-    assert Diff(a, b) < 1e-6
+    b = _reference(reflib, key + "undo", Z(*x.shape),
+                   lambda lib, b: lib.rnormUndo(dy, x, b, nf, sizeF, 0.005, 0.75, blocked), exact=False)
+    assert golden_ref.diff(a, b) < 1e-6
