@@ -54,7 +54,7 @@ void conv_up(const ConvGeom& g, const float* images, const float* filters, float
   fuse.dropped = &dropped;
   if (!(state().precision != kPrecFP32 && tc_conv_up(g, images, filters, targets, st, so, fuse))) {
     simt_conv_up(g, images, filters, targets, st, so, fuse);
-    state().last_conv_path = kPathSimt;
+    note_conv(kPathSimt, 0);
   }
   if (fuse.drop_scale != 0.f && !dropped) {        // the kernel could not apply the dropout: one pass, which also (re)writes the bf16 twin
     dropout_apply(targets, g.out_total, fuse.drop_prob, fuse.drop_scale, fuse.drop_seed, emit.buf);
@@ -78,7 +78,7 @@ void conv_down(const ConvGeom& g, const float* derivs, const float* filters, flo
   if (!late_mask) emit.attach(fuse);               // a late mask changes the values after the kernel: convert afterwards
   if (!(state().precision != kPrecFP32 && tc_conv_down(g, derivs, filters, targets, st, so, fuse))) {
     simt_conv_down(g, derivs, filters, targets, st, so, fuse);
-    state().last_conv_path = kPathSimt;
+    note_conv(kPathSimt, 0);
   }
   if (late_mask) {
     const long long n4 = g.img_total;             // (cnb_relu_deriv would consume a pending fuse request; none is pending here)
@@ -105,12 +105,12 @@ void conv_outp(const ConvGeom& g, const float* images, const float* derivs, floa
   take_fuse();                                 // a wgrad call has no epilogue to fuse: a pending request must not leak to a later call
   if (!g.conv) {                               // untied: one [Cout x K] block per module
     simt_conv_outp(g, images, derivs, targets, 1, 1, true, st, so);
-    state().last_conv_path = kPathSimt;
+    note_conv(kPathSimt, 0);
     return;
   }
   if (state().precision != kPrecFP32 && tc_conv_outp(g, images, derivs, targets, st, so)) return;
   simt_outp_auto(g, images, derivs, targets, st, so);
-  state().last_conv_path = kPathSimt;
+  note_conv(kPathSimt, 0);
 }
 
 void do_conv_up(const char* what, cudamat* images, cudamat* filters, cudamat* targets, Shape4D* is, Shape4D* fs,
@@ -358,7 +358,7 @@ void convOutp(cudamat* images, cudamat* derivs, cudamat* targets, Shape4D* is, S
   CNB_REQUIRE(targets->size[0] == g.Cout && (long long)targets->size[1] == (long long)g.K * chunks, "convOutp");
   simt_conv_outp(g, images->data_device, derivs->data_device, targets->data_device, partialSumY, partialSumX, true,
                  scaleTargets, scaleOutput);
-  state().last_conv_path = kPathSimt;
+  note_conv(kPathSimt, 0);
 }
 void localOutp(cudamat* images, cudamat* derivs, cudamat* targets, Shape4D* is, Shape4D* ds, Shape4D* ts, ConvDesc d,
                float scaleTargets, float scaleOutput) {

@@ -83,6 +83,17 @@ inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 // ---- global state (one host thread per process/GPU, like the reference) -------------
 enum Precision { kPrecFP32 = 0, kPrecTF32 = 1, kPrecBF16 = 2 };
 enum ConvPath { kPathNone = -1, kPathSimt = 0, kPathTcTf32 = 1, kPathTcBf16 = 2 };
+// which tensor-core kernel variant the last conv call ran (convnet_b200_last_conv_kernel); 0 for the CUDA-core path
+enum ConvKernelBits {
+  kKernLean = 1,              // tc_fast_kernel (else the general tc_conv_kernel)
+  kKernPair = 2,              // CTA-pair mode (in any launch of the call)
+  kKernXMode = 4,             // taps in the K block (Cin < 8)
+  kKernSplit = 8,             // K split (fprop / dgrad + reduce_split) or reduction split (wgrad + reduce_partials)
+  kKernDgradAsFprop = 16,     // dgrad as stride-1 fprop per stride phase; bits 8.. hold the phase count
+  kKernAMerged = 32,          // fprop / dgrad: merged (image-fastest) A tensor map
+  kKernBMerged = 64,          // fprop / dgrad: merged B tensor map
+};
+constexpr int kKernPhaseShift = 8;
 
 // one-shot epilogue fusion requested for the next conv / pool-undo call (convnet_b200_fuse_next)
 struct Fuse {
@@ -110,6 +121,7 @@ struct State {
   cudaStream_t stream = 0;          // legacy default stream, like every reference kernel
   int precision = kPrecFP32;      // the raw C ABI computes in fp32 (the reference's arithmetic) until a caller opts into tf32 / bf16
   int last_conv_path = kPathNone;
+  int last_conv_kernel = -1;        // ConvKernelBits of the same call
   unsigned long long launches = 0;  // kernels launched by this library
   // scratch (wgrad partial sums, rnorm-free) — grown on demand, never per-call malloc'd
   void* ws = nullptr;
@@ -128,6 +140,7 @@ int num_sms();
 inline int current_device() { int d = 0; CNB_CUDA_CHECK(cudaGetDevice(&d)); return d; }
 
 inline void count_launch(int n = 1) { state().launches += n; }
+inline void note_conv(int path, int kernel) { state().last_conv_path = path; state().last_conv_kernel = kernel; }
 inline Fuse take_fuse() { Fuse f = state().fuse; state().fuse = Fuse(); return f; }
 
 template <typename T>

@@ -53,7 +53,8 @@ struct DgradPhase {
 };
 struct DgradBanks { int count; DgradPhase phase[kMaxDgradPhases]; };
 int dgrad_phases(const ConvGeom& g, DgradBanks* b);                    // number of phases, or -1 if there are too many
-const __nv_bfloat16* dgrad_weights(const float* filters, const ConvGeom& g, const DgradBanks& b);   // built on first use, cached
+// the banks of `filters`: cached ones when valid, else built now; `keep`: they stay cached (prestage), else they serve this call only
+const __nv_bfloat16* dgrad_weights(const float* filters, const ConvGeom& g, const DgradBanks& b, bool keep);
 // max-pool tie masks (stage.cu), see pool.cu
 uint16_t* pool_masks_slot(const float* acts, long long n_out, const float* images, long long n_in, unsigned long long sig);
 const uint16_t* pool_masks_find(const float* acts, long long n_out, const float* images, unsigned long long sig);

@@ -1472,6 +1472,7 @@ static bool tc_conv_up_impl(const ConvGeom& g, const float* images, const float*
     }
   }
   bool done = false;
+  int kern = 0;
   // the lean kernel takes the shapes the training step lives in (see tc_fast_kernel); the rest stays on the general one
   if (bf && fast_enabled() && !x_mode && p.a_merged && p.splits == 1 && st == 0.f && g.Cout % 32 == 0 && p.BN % 32 == 0) {
     TcParams f = p;
@@ -1499,6 +1500,7 @@ static bool tc_conv_up_impl(const ConvGeom& g, const float* images, const float*
         if (drop) { f.drop_prob = fuse.drop_prob; f.drop_scale = fuse.drop_scale; f.drop_seed = fuse.drop_seed; }
         launch_fast<kFprop>(fa, fb, f);
         done = true;
+        kern = kKernLean | kKernAMerged | (f.cta2 ? kKernPair : 0) | (f.b_merged ? kKernBMerged : 0);
         if (drop && fuse.dropped) *fuse.dropped = true;
       }
     }
@@ -1520,12 +1522,17 @@ static bool tc_conv_up_impl(const ConvGeom& g, const float* images, const float*
     if (stages >= 2 && make_map(&fa, img, e, 5, adims, astr, abox, true) && make_map(&fb, flt, e, 5, bdims, bstr, bbox, true)) {
       launch_fast<kFprop, true>(fa, fb, f);
       done = true;
+      kern = kKernLean | kKernXMode | kKernAMerged | kKernBMerged;   // both operands through the o-chunked 5-D views
     }
   }
-  if (!done) launch<kFprop>(ma, mb, p);
+  if (!done) {
+    launch<kFprop>(ma, mb, p);
+    kern = (p.cta2 ? kKernPair : 0) | (x_mode ? kKernXMode : 0) | (p.splits > 1 ? kKernSplit : 0) |
+           (p.a_merged ? kKernAMerged : 0) | (p.b_merged ? kKernBMerged : 0);
+  }
   if (emit && fuse.emitted) *fuse.emitted = true;
   if (p.splits > 1) reduce_split((const float*)ws, out, out_elems, p.splits, st, so, bias, (long long)g.modules * g.N, fuse.relu, nullptr);
-  state().last_conv_path = bf ? kPathTcBf16 : kPathTcTf32;
+  note_conv(bf ? kPathTcBf16 : kPathTcTf32, kern);
   return true;
 }
 bool tc_conv_up(const ConvGeom& g, const float* images, const float* filters, float* targets, float st, float so,
@@ -1558,7 +1565,7 @@ static bool dgrad_as_fprop_eligible(const ConvGeom& g, const float* derivs, cons
 void tc_conv_down_prestage(const ConvGeom& g, const float* derivs, const float* filters) {
   DgradBanks banks;
   if (!tc_enabled() || !g.conv || !want_bf16() || !dgrad_as_fprop_eligible(g, derivs, filters, &banks)) return;
-  dgrad_weights(filters, g, banks);
+  dgrad_weights(filters, g, banks, true);
 }
 
 static bool tc_conv_down_as_fprop(const ConvGeom& g, const float* derivs, const float* filters, float* targets, float so,
@@ -1573,8 +1580,9 @@ static bool tc_conv_down_as_fprop(const ConvGeom& g, const float* derivs, const 
     to_bf16(derivs, tmp, g.out_total);
     sd = tmp;
   }
-  const __nv_bfloat16* bank = dgrad_weights(filters, g, banks);
+  const __nv_bfloat16* bank = dgrad_weights(filters, g, banks, false);
   bool emitted_all = fuse.out16 != nullptr;
+  int kern = kKernDgradAsFprop | kKernLean | kKernAMerged | (banks.count << kKernPhaseShift);
   for (int i = 0; i < banks.count; i++) {
     const DgradPhase& P = banks.phase[i];
     TcParams p; fill_common(p, g, e);
@@ -1617,9 +1625,10 @@ static bool tc_conv_down_as_fprop(const ConvGeom& g, const float* derivs, const 
     }
     if (!ok) { CNB_REQUIRE(i == 0, "dgrad-as-fprop: tensor map failed after the first phase"); return false; }
     launch_fast<kFprop>(fa, fb, p);
+    kern |= (p.cta2 ? kKernPair : 0) | (p.b_merged ? kKernBMerged : 0);
   }
   if (emitted_all && fuse.emitted) *fuse.emitted = true;
-  state().last_conv_path = kPathTcBf16;
+  note_conv(kPathTcBf16, kern);
   return true;
 }
 
@@ -1701,7 +1710,8 @@ static bool tc_conv_down_impl(const ConvGeom& g, const float* derivs, const floa
       launch<kDgrad>(ma, mb, p);
     }
   }
-  state().last_conv_path = bf ? kPathTcBf16 : kPathTcTf32;
+  note_conv(bf ? kPathTcBf16 : kPathTcTf32,
+            (p.cta2 ? kKernPair : 0) | (p.splits > 1 ? kKernSplit : 0) | (p.a_merged ? kKernAMerged : 0));
   return true;
 }
 bool tc_conv_down(const ConvGeom& g, const float* derivs, const float* filters, float* targets, float st, float so,
@@ -1797,6 +1807,7 @@ static bool tc_conv_outp_impl(const ConvGeom& g, const float* images, const floa
   } else if (!image_map(&mb, img, e, g, g.W, g.H, g.Cin, g.in_frame_step, false, bn_local)) return false;
   p.out = p.splits == 1 ? targets : (float*)ws;
   bool done = false;
+  int kern = (p.cta2 ? kKernPair : 0) | (x_mode ? kKernXMode : 0) | (p.splits > 1 ? kKernSplit : 0);
   if (bf && fast_enabled() && !x_mode && g.frames == 1 && g.N % 128 == 0 && g.Cin % 32 == 0 && p.BN % 32 == 0 &&
       (p.splits > 1 || st == 0.f)) {
     TcParams f = p;
@@ -1812,6 +1823,7 @@ static bool tc_conv_outp_impl(const ConvGeom& g, const float* images, const floa
       if (make_map(&fa, der, e, 5, adims, astr, abox, false) && make_map(&fb, img, e, 5, bdims, bstr, bbox, false)) {
         launch_fast<kWgrad>(fa, fb, f);
         done = true;
+        kern |= kKernLean;
       }
     }
   }
@@ -1834,11 +1846,12 @@ static bool tc_conv_outp_impl(const ConvGeom& g, const float* images, const floa
     if (stages >= 2 && make_map(&fa, der, e, 5, adims, astr, abox, false) && make_map(&fb, img, e, 5, bdims, bstr, bbox, false)) {
       launch_fast<kWgrad, true>(fa, fb, f);
       done = true;
+      kern |= kKernLean;
     }
   }
   if (!done) launch<kWgrad>(ma, mb, p);
   if (p.splits > 1) reduce_partials((const float*)ws, targets, elems, 1, p.splits, st, so);
-  state().last_conv_path = bf ? kPathTcBf16 : kPathTcTf32;
+  note_conv(bf ? kPathTcBf16 : kPathTcTf32, kern);
   return true;
 }
 bool tc_conv_outp(const ConvGeom& g, const float* images, const float* derivs, float* targets, float st, float so) {

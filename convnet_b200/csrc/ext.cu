@@ -109,6 +109,7 @@ void convnet_b200_bf16_ensure(const float* ptr, long long n) { bf16_ensure(ptr, 
 int convnet_b200_bf16_is_staged(const float* ptr, long long n) { return want_bf16() && bf16_staged(ptr, n) != nullptr; }
 void convnet_b200_bf16_invalidate(const float* ptr) { bf16_invalidate(ptr); }
 int convnet_b200_last_conv_path(void) { return state().last_conv_path; }
+int convnet_b200_last_conv_kernel(void) { return state().last_conv_kernel; }
 unsigned long long convnet_b200_launch_count(void) { return state().launches; }
 void convnet_b200_reset_launch_count(void) { state().launches = 0; }
 void convnet_b200_release_workspace(void) {

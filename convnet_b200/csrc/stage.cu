@@ -122,7 +122,7 @@ Staged* acquire_slot(const float* ptr, long long n, int kind = 0) {
 // form it uses the fprop kernel (CTA pairs, MN-major B), which needs the filters of a phase as [c fastest][tap''][o]:
 //   bank(a,b)[c + Cin*((u' + ku*v') + ku*kv*o)] = w[o, tx = ra + sx*(ku-1-u'), ty = rb + sy*(kv-1-v'), c]
 // (reference semantics: cudamat_conv_gemm.cu:684-825, convDown = Sgemm + kContract).  The banks are a permutation of the
-// filter tensor (every tap belongs to exactly one phase), built by one small kernel and cached like a bf16 copy.
+// filter tensor (every tap belongs to exactly one phase), built by one small kernel; cached like a bf16 copy when prestaged.
 // one 32 x 32 (o, c) tile of one tap per block: coalesced reads along o, coalesced writes along c
 __global__ void __launch_bounds__(256) dgrad_bank_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ out, DgradBanks b,
                                                          int Cin, int Cout, int kx, int ky, int sx, int sy) {
@@ -170,7 +170,11 @@ int dgrad_phases(const ConvGeom& g, DgradBanks* b) {
   return b->count;
 }
 
-const __nv_bfloat16* dgrad_weights(const float* filters, const ConvGeom& g, const DgradBanks& b) {
+// Only banks built on request (convnet_b200_prestage_next: `keep`) stay valid after the call.  Like a staged copy, cached
+// banks follow library writes to the filters but not writes the library cannot see, and a caller that overwrites its
+// weights by other means (its own optimizer, a cudaMemcpy) never asked to cache anything: banks built inside a convDown
+// serve that call alone.  Their buffer stays with the slot, so the next such call rebuilds into it in stream order.
+const __nv_bfloat16* dgrad_weights(const float* filters, const ConvGeom& g, const DgradBanks& b, bool keep) {
   const long long n = (long long)g.Cout * g.K;
   unsigned long long sig = 1469598103934665603ULL;
   for (int v : {g.Cin, g.Cout, g.kx, g.ky, g.sx, g.sy, g.px, g.py, g.W, g.H}) sig = (sig ^ (unsigned)v) * 1099511628211ULL;
@@ -182,7 +186,7 @@ const __nv_bfloat16* dgrad_weights(const float* filters, const ConvGeom& g, cons
   dgrad_bank_kernel<<<grid, 256, 0, state().stream>>>(filters, e->buf, b, g.Cin, g.Cout, g.kx, g.ky, g.sx, g.sy);
   count_launch();
   CNB_LAUNCH_CHECK("dgrad_banks");
-  e->valid = true; e->sig = sig;
+  e->valid = keep; e->sig = sig;
   return e->buf;
 }
 

@@ -70,6 +70,7 @@ SIGNATURES = {
     "convnet_b200_set_conv_precision": [I],
     "convnet_b200_get_conv_precision": [],
     "convnet_b200_last_conv_path": [],
+    "convnet_b200_last_conv_kernel": [],
     "convnet_b200_launch_count": [],
     "convnet_b200_fuse_next": [FP, I, FP],
     "convnet_b200_bf16_stage": [FP, ct.c_longlong],
@@ -101,7 +102,8 @@ SIGNATURES = {
 }
 RESTYPES = {
     "convnet_b200_version": I, "convnet_b200_get_stream": ct.c_void_p,
-    "convnet_b200_get_conv_precision": I, "convnet_b200_last_conv_path": I, "convnet_b200_bf16_is_staged": I,
+    "convnet_b200_get_conv_precision": I, "convnet_b200_last_conv_path": I, "convnet_b200_last_conv_kernel": I,
+    "convnet_b200_bf16_is_staged": I,
     "convnet_b200_launch_count": ct.c_ulonglong, "convnet_b200_extract_patches": I,
 }
 
@@ -135,3 +137,15 @@ def set_precision(mode):
 
 def last_conv_path():
     return PATH_NAME[load().convnet_b200_last_conv_path()]
+
+
+KERNEL_BITS = {"lean": 1, "pair": 2, "xmode": 4, "split": 8, "dgrad_as_fprop": 16, "a_merged": 32, "b_merged": 64}
+
+
+def last_conv_kernel():
+    """the variant the last conv call ran (convnet_b200_last_conv_kernel): the set of KERNEL_BITS names plus the number
+    of stride phases of a dgrad-as-fprop call, or None before the first call"""
+    v = load().convnet_b200_last_conv_kernel()
+    if v < 0:
+        return None
+    return {name for name, bit in KERNEL_BITS.items() if v & bit}, v >> 8

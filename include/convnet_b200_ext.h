@@ -38,6 +38,14 @@ int convnet_b200_get_conv_precision(void);
  * 2 tcgen05 bf16, -1 none yet.  (tests assert the tensor path really ran) */
 int convnet_b200_last_conv_path(void);
 
+/* Which kernel variant the most recent conv call ran, as a bit mask (0 for the CUDA-core path, -1 none yet).  It only
+ * records what the shape and the mode selected; tests use it to prove a case reaches the variant it exists for.
+ *   1 lean kernel          2 CTA pair (in any launch of the call)      4 x-mode (Cin < 8: filter taps in the K block)
+ *   8 K split (fprop / dgrad) or reduction split (wgrad) > 1           16 dgrad run as stride-1 fprop per stride phase
+ *   32 merged A tensor map (fprop / dgrad)                             64 merged B tensor map (fprop / dgrad)
+ *   bits 8..12: number of stride phases of a dgrad-as-fprop call */
+int convnet_b200_last_conv_kernel(void);
+
 /* Number of kernels this library has launched since the last reset. */
 unsigned long long convnet_b200_launch_count(void);
 void convnet_b200_reset_launch_count(void);

@@ -54,6 +54,7 @@ def test_ctypes_signatures_cover_every_declared_symbol(libpath):
     assert L.convnet_b200_version() >= 100
     assert L.convnet_b200_get_conv_precision() in (0, 1, 2)
     assert L.convnet_b200_last_conv_path() == -1
+    assert L.convnet_b200_last_conv_kernel() == -1
 
 
 def test_abi_struct_sizes_match_reference_layout():
